@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # the CUDA path (mcpilco_b200)
     python bench.py --impl reference [--gpus N] [--steps K] ...     # the reference algorithm on the host CPU (oracle port)
+    python bench.py --steps K --dump-outputs DIR                    # also write the last timed step's outputs, to compare two builds
 
 A "step" is what one iteration of MC_PILCO.reinforce_policy does on the hot path (reference MC_PILCO.py:484-522):
 apply_policy -> cost_function -> cost.backward(), i.e. M*H particle-steps forward and backward, including the cost, the
@@ -54,7 +55,15 @@ def parse():
     ap.add_argument("--no-forward-only", action="store_true", help="skip the forward-only (no-grad rollout) measurement")
     ap.add_argument("--cpu-particles-all", type=int, default=2048, help="cpu_baseline sample with all host threads: particles (SURVEY 8d: min(M, 2048))")
     ap.add_argument("--cpu-horizon-all", type=int, default=8, help="cpu_baseline sample with all host threads: horizon (SURVEY 8d: 8)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned (states, inputs, cost, std, policy gradients) "
+                         "as DIR/<name>.npy in float64; beyond 64 MB in all, states and inputs keep a seeded sample of the particles")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "own":
+        ap.error("--dump-outputs dumps the CUDA path (--impl own)")
+    return a
 
 
 # ------------------------------------------------------------------------------------------------------------------
@@ -380,7 +389,7 @@ def own_arm(args):
         states, inputs = obj.apply_policy(particles_initial_state_mean=mean, particles_initial_state_var=var, **kw)
         cost, std = obj.cost_function(states, inputs, 0)
         cost.backward()
-        return cost, std
+        return cost, std, states, inputs
 
     def barrier():
         if world > 1:
@@ -408,7 +417,7 @@ def own_arm(args):
         torch.cuda.profiler.start()
     e0.record()
     for _ in range(args.steps):
-        cost, std = step()
+        cost, std, states, inputs = step()
     e1.record()
     barrier()
     if args.cuda_profiler_range:
@@ -420,6 +429,11 @@ def own_arm(args):
     ops.prof_enable(False)
     cost_v = float(cost.detach())
     value = M_global * H * args.steps / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:  # under torch.distributed: rank 0's particles
+        dump_outputs(args.dump_outputs, {"states": states, "inputs": inputs, "cost": cost, "std_cost": std,
+                                         "grad_log_lengthscales": pol.log_lengthscales.grad, "grad_centers": pol.centers.grad,
+                                         "grad_weight": pol.f_linear.weight.grad}, per_particle=("states", "inputs"))
+    del states, inputs  # not held through the measurements below
 
     # ---- end to end: host buffers in, host results out, through the same public API ----
     host_in = [p.detach().cpu().pin_memory() for p in params] + [mean_d.cpu().pin_memory(), var_d.cpu().pin_memory()]
@@ -433,7 +447,7 @@ def own_arm(args):
                 p.copy_(h, non_blocking=True)
         mean = host_in[3].to(dev, non_blocking=True)
         var = host_in[4].to(dev, non_blocking=True)
-        c, s = step(mean, var)
+        c, s = step(mean, var)[:2]
         host_out[0].copy_(torch.stack([c.detach(), s.detach()]), non_blocking=True)
         for h, p in zip(host_out[1:], params):
             h.copy_(p.grad.reshape(-1), non_blocking=True)
@@ -459,7 +473,7 @@ def own_arm(args):
 
         def replay_step():
             obj._rollouts = REPLAY
-            c, _ = step()
+            c = step()[0]
             return float(c.detach()), [p.grad.detach().clone() for p in params]
 
         def grad_rel(ga, gb):
@@ -475,7 +489,7 @@ def own_arm(args):
             ops.prof_enable(True)
             e0.record()
             for _ in range(2):
-                vc, _ = step()
+                vc = step()[0]
             e1.record()
             barrier()
             vms = max_over_ranks(e0.elapsed_time(e1)) / 2
@@ -578,6 +592,26 @@ def own_arm(args):
     if world > 1:
         dist.destroy_process_group()
     return 0
+
+
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(path, arrays, per_particle):
+    """Write `arrays` (name -> tensor) as path/<name>.npy in float64.  The arrays named in `per_particle` are [H, M, ...]; when
+    everything would exceed DUMP_BYTES they keep a seeded sample of the M particles (sorted, the same for each of them and for every
+    run with the same M), so that dumps of two builds compare element for element."""
+    out = {k: v.detach().double().cpu().numpy() for k, v in arrays.items()}
+    M = out[per_particle[0]].shape[1]
+    fixed = sum(a.nbytes for k, a in out.items() if k not in per_particle) + 128 * len(out)  # + the .npy headers
+    per = sum(out[k].nbytes for k in per_particle) // M
+    if fixed + M * per > DUMP_BYTES:
+        keep = np.sort(np.random.RandomState(0).choice(M, (DUMP_BYTES - fixed) // per, replace=False))
+        for k in per_particle:
+            out[k] = out[k][:, keep]
+    os.makedirs(path, exist_ok=True)
+    for k, a in out.items():
+        np.save(os.path.join(path, k + ".npy"), a)
 
 
 def emit(line):
