@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define MCP_ABI_VERSION 6
+#define MCP_ABI_VERSION 7
 
 #define MCP_MAX_D 32    /* gp-input dimension            */
 #define MCP_MAX_DS 16   /* state dimension               */
@@ -258,6 +258,16 @@ int mcpilco_rollout_bwd(const McpRollout* r, const McpRolloutGrad* g, void* stre
  * 389-403).  `masks_t` is [M, nb] or NULL. */
 int mcpilco_policy_forward(const McpPolicy* policy, int M, int t, const double* x, double p_dropout, const uint8_t* masks_t,
                            uint64_t seed, uint64_t particle_offset, double* u, void* stream);
+
+/* Vector-Jacobian product of mcpilco_policy_forward: given g_u[M, Du] = dL/du, writes dL/dx [M, Ds] (g_x may be NULL) and
+ * dL/d{log_ls [Dp], centers [nb, Dp], W [Du, nb], bias [Du] (NULL if !has_bias)}.  The arguments mean what they mean for the
+ * forward, including the dropout mask (the same injected masks_t, or the same Philox draws for (seed, particle_offset + m, t, b)).
+ * Outputs are overwritten, not accumulated; M == 0 writes zeros.  Sums over particles are reduced in a fixed order: repeated
+ * calls on one device are bit-identical.  `workspace` holds mcpilco_policy_backward_workspace_bytes(M, nb, Dp, Du) bytes. */
+size_t mcpilco_policy_backward_workspace_bytes(int M, int nb, int Dp, int Du);
+int mcpilco_policy_backward(const McpPolicy* policy, int M, int t, const double* x, double p_dropout, const uint8_t* masks_t,
+                            uint64_t seed, uint64_t particle_offset, const double* g_u, double* g_x, double* g_log_ls,
+                            double* g_centers, double* g_W, double* g_bias, void* workspace, size_t workspace_bytes, void* stream);
 
 /* Initial particles (MC_PILCO.apply_policy, policy_learning/MC_PILCO.py:635-657) from counter-based Philox keyed by the
  * global particle id:  kind 0: x0 = a[k] + b[k] * n, n ~ N(0, I)  (a = mean, b = sqrt(var); n_modes > 1 draws the mode k

@@ -803,6 +803,164 @@ __global__ void scatter_grads_kernel(const double* __restrict__ flat, int Dp, in
 }
 
 // ------------------------------------------------------------------------------------------------
+// stand-alone policy backward: the vector-Jacobian product of mcpilco_policy_forward (Policy.py:242-265,323-335,389-403 under
+// autograd).  Threads own basis functions, as in policy_block_body; a CTA walks its particles one after the other, so that every
+// thread keeps g_centers[b, :] and g_W[:, b] in registers and the particle sums need no atomics.  Per particle:
+//   h_b (recomputed, same dropout draw as the forward) -> [squash only: u = u_max tanh((W h + bias) / u_max)] ->
+//   la = g_u (1 - (u / u_max)^2) -> g_W += la h^T, dL/dd_b = -h_b <la, W[:, b]> -> d/dz by a butterfly per warp -> warp 0: dL/dx.
+// The log-lengthscale gradient uses the identity of rollout_bwd_kernel: g_logls_j = -sum z_j lz_j - sum_b c_bj g_c[b][j].
+// ------------------------------------------------------------------------------------------------
+template <int DPT, int DUT>
+__global__ void __launch_bounds__(512) policy_bwd_kernel(const __grid_constant__ McpPolicy pol, const __grid_constant__ McpNoise nz, int M, int t,
+                                                         const double* __restrict__ x, const double* __restrict__ g_u,
+                                                         double* __restrict__ g_x, double* __restrict__ partials) {
+  extern __shared__ double s_cb[];  // [Dp][blockDim.x] centres, then [Du][blockDim.x] weights of each thread's basis function
+  __shared__ double s_il[MCP_MAX_DP], s_z[MCP_MAX_DP];
+  __shared__ double s_part[16][MCP_MAX_DU], s_la[MCP_MAX_DU];
+  __shared__ double s_red[16][MCP_MAX_DP];
+  const int nb = pol.nb, Dp = pol.Dp, Du = pol.Du, Ds = pol.Ds;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nw = blockDim.x >> 5, nthr = blockDim.x;
+  const int b = tid;
+  const bool has_b = b < nb;
+  if (tid < Dp) s_il[tid] = exp(-pol.log_ls[tid]);
+  double* const s_wb = s_cb + (size_t)Dp * nthr;
+  double gc[DPT], gw[DUT];
+#pragma unroll
+  for (int j = 0; j < DPT; j++) {
+    if (j < Dp) s_cb[(size_t)j * nthr + tid] = has_b ? pol.centers[(size_t)b * Dp + j] : 0.0;
+    gc[j] = 0.0;
+  }
+#pragma unroll
+  for (int k = 0; k < DUT; k++) {
+    if (k < Du) s_wb[(size_t)k * nthr + tid] = has_b ? pol.W[(size_t)k * nb + b] : 0.0;
+    gw[k] = 0.0;
+  }
+  const bool drop = dropout_active(pol, nz);
+  const double keep_scale = drop ? 1.0 / (1.0 - nz.p_dropout) : 1.0;
+  // warp 0: lane j carries the log-lengthscale gradient j (first half), lane k the bias gradient k; and where state component `lane`
+  // sits in the feature lists (-1: nowhere)
+  double glz = 0.0, gbias = 0.0;
+  int c_pna = -1, c_pa = -1;
+  if (warp == 0 && pol.kind == 1) {
+    for (int i = 0; i < pol.n_na; i++) if (pol.na_idx[i] == lane) c_pna = i;
+    for (int i = 0; i < pol.n_a; i++) if (pol.a_idx[i] == lane) c_pa = i;
+  }
+  __syncthreads();
+
+  for (int m = blockIdx.x; m < M; m += gridDim.x) {
+    const double* xm = x + (size_t)m * Ds;
+    if (tid < Dp) s_z[tid] = policy_feature(pol, xm, t, tid);
+    __syncthreads();
+    double h = 0.0;
+    if (has_b) {
+      double d = 0.0;
+#pragma unroll 4
+      for (int j = 0; j < Dp; j++) { const double q = (s_z[j] - s_cb[(size_t)j * nthr + tid]) * s_il[j]; d = fma(q, q, d); }
+      h = exp(-d);
+      if (drop) h = keep_unit(nz, M, nb, 0, t, m, b) ? h * keep_scale : 0.0;
+    }
+    if (pol.squash) {  // the squash derivative needs the forward output
+#pragma unroll
+      for (int k = 0; k < DUT; k++)
+        if (k < Du) {
+          const double v = warp_sum(s_wb[(size_t)k * nthr + tid] * h);
+          if (lane == 0) s_part[warp][k] = v;
+        }
+    }
+    __syncthreads();
+    if (tid < Du) {
+      double la = g_u[(size_t)m * Du + tid];
+      if (pol.squash) {
+        double v = 0.0;
+        for (int i = 0; i < nw; i++) v += s_part[i][tid];  // fixed order
+        if (pol.has_bias) v += pol.bias[tid];
+        const double q = tanh(v / pol.u_max[tid]);
+        la *= 1.0 - q * q;
+      }
+      s_la[tid] = la;
+      gbias += la;
+    }
+    __syncthreads();
+    double lh = 0.0;
+#pragma unroll
+    for (int k = 0; k < DUT; k++)
+      if (k < Du) { gw[k] = fma(s_la[k], h, gw[k]); lh = fma(s_la[k], s_wb[(size_t)k * nthr + tid], lh); }
+    const double ld_b = -h * lh;  // dL/dd_b
+#pragma unroll
+    for (int j0 = 0; j0 < DPT; j0 += 8) {
+      double cz[8];
+#pragma unroll
+      for (int jj = 0; jj < 8; jj++) {
+        const int j = j0 + jj;
+        cz[jj] = (j < Dp) ? ld_b * 2.0 * (s_z[j] - s_cb[(size_t)j * nthr + tid]) * s_il[j] * s_il[j] : 0.0;  // d/dz_j ; d/dc_bj = -cz
+        gc[j] -= cz[jj];
+      }
+      warp_sum_multi<8>(cz, lane);
+      if ((lane & 3) == 0 && j0 + (lane >> 2) < Dp) s_red[warp][j0 + (lane >> 2)] = cz[0];
+    }
+    __syncthreads();
+    if (warp == 0) {
+      double lz = 0.0;  // dL/dz_lane
+      if (lane < Dp) {
+        for (int w2 = 0; w2 < nw; w2++) lz += s_red[w2][lane];
+        glz -= s_z[lane] * lz;
+      }
+      if (g_x != nullptr) {
+        double gx = 0.0;
+        if (pol.kind == 1) {
+          const int n_na = pol.n_na, n_a = pol.n_a;
+          const double z_na = __shfl_sync(0xffffffffu, lz, c_pna >= 0 ? c_pna : 0);
+          const double z_c = __shfl_sync(0xffffffffu, lz, (n_na + (c_pa >= 0 ? c_pa : 0)) & 31);
+          const double z_s = __shfl_sync(0xffffffffu, lz, (n_na + n_a + (c_pa >= 0 ? c_pa : 0)) & 31);
+          if (c_pna >= 0) gx += z_na * pol.inv_scale[c_pna];
+          if (c_pa >= 0) {
+            double sn, cs;
+            sincos(xm[lane], &sn, &cs);
+            gx += -z_c * pol.inv_scale[n_na + c_pa] * sn + z_s * pol.inv_scale[n_na + n_a + c_pa] * cs;
+          }
+        } else if (pol.kind == 2) {
+          const double z_t = __shfl_sync(0xffffffffu, lz, (Ds + lane) & 31);
+          if (lane < Ds) gx = lz * pol.inv_scale[lane] - z_t * pol.inv_scale[Ds + lane];
+        } else if (lane < Ds) {
+          gx = lz * pol.inv_scale[lane];
+        }
+        if (lane < Ds) g_x[(size_t)m * Ds + lane] = gx;
+      }
+      __syncwarp();
+    }
+  }
+
+  // per-CTA partials in the layout of reduce_partials_kernel / scatter_grads_kernel: [g_log_ls | g_centers | g_W | g_bias]
+  double* P = partials + (size_t)blockIdx.x * (Dp + (size_t)nb * Dp + (size_t)Du * nb + Du);
+  __syncthreads();
+#pragma unroll
+  for (int j0 = 0; j0 < DPT; j0 += 8) {
+    double cg[8];
+#pragma unroll
+    for (int jj = 0; jj < 8; jj++) cg[jj] = (j0 + jj < Dp) ? s_cb[(size_t)(j0 + jj) * nthr + tid] * gc[j0 + jj] : 0.0;
+    warp_sum_multi<8>(cg, lane);
+    if ((lane & 3) == 0 && j0 + (lane >> 2) < Dp) s_red[warp][j0 + (lane >> 2)] = cg[0];
+  }
+  __syncthreads();
+  if (warp == 0) {
+    if (lane < Dp) {
+      double v = 0.0;
+      for (int w2 = 0; w2 < nw; w2++) v += s_red[w2][lane];
+      P[lane] = glz - v;
+    }
+    if (lane < Du) P[Dp + (size_t)nb * Dp + (size_t)Du * nb + lane] = gbias;
+  }
+  if (has_b) {
+#pragma unroll
+    for (int j = 0; j < DPT; j++)
+      if (j < Dp) P[Dp + (size_t)b * Dp + j] = gc[j];
+#pragma unroll
+    for (int k = 0; k < DUT; k++)
+      if (k < Du) P[Dp + (size_t)nb * Dp + (size_t)k * nb + b] = gw[k];
+  }
+}
+
+// ------------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------------
 struct Workspace {
@@ -904,6 +1062,32 @@ static int check_rollout(const McpRollout* r) {
   MCP_CHECK_ARG(r->noise.p_dropout >= 0.0 && r->noise.p_dropout < 1.0, "rollout: p_dropout outside [0,1)");
   for (int e = 0; e < m.E; e++) MCP_CHECK_ARG(r->gps[e].spec.D == m.D, "rollout: gp %d input dim %d != %d", e, r->gps[e].spec.D, m.D);
   return MCP_OK;
+}
+
+// argument checks shared by the stand-alone policy forward and backward
+static int check_policy_call(const McpPolicy* policy, int M, double p_dropout, const char* fn) {
+  MCP_CHECK_ARG(policy != nullptr && M >= 0, "%s: null policy", fn);
+  const McpPolicy& p = *policy;
+  MCP_CHECK_ARG(p.nb >= 1 && p.nb <= 512 && p.Dp >= 1 && p.Dp <= MCP_MAX_DP && p.Du >= 1 && p.Du <= MCP_MAX_DU && p.Ds >= 1 && p.Ds <= MCP_MAX_DS,
+                "%s: policy dims out of range (nb=%d Dp=%d Du=%d Ds=%d)", fn, p.nb, p.Dp, p.Du, p.Ds);
+  int dp = p.kind == 1 ? p.n_na + 2 * p.n_a : (p.kind == 2 ? 2 * p.Ds : p.Ds);
+  MCP_CHECK_ARG(dp == p.Dp, "%s: feature dimension %d does not match kind %d (%d)", fn, p.Dp, p.kind, dp);
+  MCP_CHECK_ARG(p.log_ls && p.centers && p.W && (!p.has_bias || p.bias) && (p.kind != 2 || p.target_traj), "%s: null policy tensor", fn);
+  MCP_CHECK_ARG(p_dropout >= 0.0 && p_dropout < 1.0, "%s: p_dropout outside [0,1)", fn);
+  return MCP_OK;
+}
+
+static int policy_bwd_threads(int nb) { return (nb + 31) / 32 * 32; }
+
+// CTAs of the policy backward: about 1024 resident threads per SM, at most one CTA per particle
+static int policy_bwd_ctas(int M, int nb) {
+  int sms = 148;
+  int dev = 0;
+  if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  int per_sm = 1024 / policy_bwd_threads(nb);
+  per_sm = per_sm < 1 ? 1 : (per_sm > 8 ? 8 : per_sm);
+  const int g = sms * per_sm;
+  return M < g ? M : g;
 }
 
 }  // namespace mcp
@@ -1060,14 +1244,7 @@ extern "C" __attribute__((visibility("default"))) int mcpilco_rollout_bwd(const 
 extern "C" __attribute__((visibility("default"))) int mcpilco_policy_forward(const McpPolicy* policy, int M, int t, const double* x, double p_dropout,
                                                                               const uint8_t* masks_t, uint64_t seed, uint64_t particle_offset,
                                                                               double* u, void* stream) {
-  MCP_CHECK_ARG(policy != nullptr && M >= 0, "policy_forward: null policy");
-  const McpPolicy& p = *policy;
-  MCP_CHECK_ARG(p.nb >= 1 && p.nb <= 512 && p.Dp >= 1 && p.Dp <= MCP_MAX_DP && p.Du >= 1 && p.Du <= MCP_MAX_DU && p.Ds >= 1 && p.Ds <= MCP_MAX_DS,
-                "policy_forward: policy dims out of range (nb=%d Dp=%d Du=%d Ds=%d)", p.nb, p.Dp, p.Du, p.Ds);
-  int dp = p.kind == 1 ? p.n_na + 2 * p.n_a : (p.kind == 2 ? 2 * p.Ds : p.Ds);
-  MCP_CHECK_ARG(dp == p.Dp, "policy_forward: feature dimension %d does not match kind %d (%d)", p.Dp, p.kind, dp);
-  MCP_CHECK_ARG(p.log_ls && p.centers && p.W && (!p.has_bias || p.bias) && (p.kind != 2 || p.target_traj), "policy_forward: null policy tensor");
-  MCP_CHECK_ARG(p_dropout >= 0.0 && p_dropout < 1.0, "policy_forward: p_dropout outside [0,1)");
+  if (int e = check_policy_call(policy, M, p_dropout, "policy_forward")) return e;
   if (M == 0) return MCP_OK;
   MCP_CHECK_ARG(x && u, "policy_forward: null state / input buffer");
   McpModel mdl{};
@@ -1076,7 +1253,60 @@ extern "C" __attribute__((visibility("default"))) int mcpilco_policy_forward(con
   nz.seed = seed;
   nz.particle_offset = particle_offset;
   nz.p_dropout = p_dropout;
-  return launch_policy(p, mdl, nz, M, M, t, 0, x, x, u, nullptr, (cudaStream_t)stream);
+  return launch_policy(*policy, mdl, nz, M, M, t, 0, x, x, u, nullptr, (cudaStream_t)stream);
+}
+
+extern "C" __attribute__((visibility("default"))) size_t mcpilco_policy_backward_workspace_bytes(int M, int nb, int Dp, int Du) {
+  const size_t nparam = (size_t)Dp + (size_t)nb * Dp + (size_t)Du * nb + Du;
+  const int ctas = policy_bwd_ctas(M > 0 ? M : 1, nb);
+  return (align_up((size_t)ctas * nparam, 32) + nparam) * sizeof(double) + 256;
+}
+
+extern "C" __attribute__((visibility("default"))) int mcpilco_policy_backward(const McpPolicy* policy, int M, int t, const double* x, double p_dropout,
+                                                                               const uint8_t* masks_t, uint64_t seed, uint64_t particle_offset,
+                                                                               const double* g_u, double* g_x, double* g_log_ls, double* g_centers,
+                                                                               double* g_W, double* g_bias, void* workspace, size_t workspace_bytes,
+                                                                               void* stream) {
+  if (int e = check_policy_call(policy, M, p_dropout, "policy_backward")) return e;
+  const McpPolicy& p = *policy;
+  MCP_CHECK_ARG(g_log_ls && g_centers && g_W && (!p.has_bias || g_bias), "policy_backward: null gradient output");
+  cudaStream_t st = (cudaStream_t)stream;
+  const int nb = p.nb, Dp = p.Dp, Du = p.Du;
+  if (M == 0) {
+    MCP_CUDA(cudaMemsetAsync(g_log_ls, 0, sizeof(double) * Dp, st));
+    MCP_CUDA(cudaMemsetAsync(g_centers, 0, sizeof(double) * (size_t)nb * Dp, st));
+    MCP_CUDA(cudaMemsetAsync(g_W, 0, sizeof(double) * (size_t)Du * nb, st));
+    if (p.has_bias) MCP_CUDA(cudaMemsetAsync(g_bias, 0, sizeof(double) * Du, st));
+    return MCP_OK;
+  }
+  MCP_CHECK_ARG(x && g_u, "policy_backward: null state / gradient buffer");
+  MCP_CHECK_ARG(workspace && workspace_bytes >= mcpilco_policy_backward_workspace_bytes(M, nb, Dp, Du), "policy_backward: workspace too small");
+  const int nparam = Dp + nb * Dp + Du * nb + Du;
+  const int ctas = policy_bwd_ctas(M, nb), threads = policy_bwd_threads(nb);
+  double* partials = (double*)align_up((size_t)workspace, 256);
+  double* flat = partials + align_up((size_t)ctas * nparam, 32);
+  McpNoise nz{};
+  nz.masks = masks_t;
+  nz.seed = seed;
+  nz.particle_offset = particle_offset;
+  nz.p_dropout = p_dropout;
+  const size_t smem = (size_t)(Dp + Du) * threads * sizeof(double);  // <= 160 KB
+#define MCP_PBWD(DPT, DUT)                                                                              \
+  do {                                                                                                  \
+    static bool cfg_[MCP_MAX_DEVICES] = {};                                                             \
+    MCP_CUDA(ensure_dynamic_smem(cfg_, policy_bwd_kernel<DPT, DUT>, 160 * 1024));                       \
+    policy_bwd_kernel<DPT, DUT><<<ctas, threads, smem, st>>>(p, nz, M, t, x, g_u, g_x, partials);       \
+  } while (0)
+  if (Dp <= 8) { if (Du <= 2) MCP_PBWD(8, 2); else MCP_PBWD(8, 8); }
+  else if (Dp <= 16) { if (Du <= 2) MCP_PBWD(16, 2); else MCP_PBWD(16, 8); }
+  else { if (Du <= 2) MCP_PBWD(32, 2); else MCP_PBWD(32, 8); }
+#undef MCP_PBWD
+  MCP_LAUNCH_CHECK();
+  reduce_partials_kernel<<<cdiv(nparam, 128), 128, 0, st>>>(partials, ctas, nparam, flat);
+  MCP_LAUNCH_CHECK();
+  scatter_grads_kernel<<<cdiv(nparam, 128), 128, 0, st>>>(flat, Dp, nb, Du, g_log_ls, g_centers, g_W, p.has_bias ? g_bias : nullptr);
+  MCP_LAUNCH_CHECK();
+  return MCP_OK;
 }
 
 extern "C" __attribute__((visibility("default"))) int mcpilco_init_particles(int kind, const double* a, const double* b, int n_modes, int M, int Ds,

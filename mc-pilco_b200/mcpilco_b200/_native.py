@@ -6,7 +6,7 @@ import ctypes as C
 import os
 
 MAX_D, MAX_DS, MAX_DU, MAX_E, MAX_DP, MAX_POLY, MAX_DEG = 32, 16, 8, 16, 32, 3, 3
-ABI_VERSION = 6
+ABI_VERSION = 7
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libmcpilco_b200.so")
 
@@ -94,6 +94,10 @@ SYMBOLS = {
     "mcpilco_rollout_bwd": (C.c_int, [C.POINTER(Rollout), C.POINTER(RolloutGrad), C.c_void_p]),
     "mcpilco_policy_forward": (C.c_int, [C.POINTER(Policy), C.c_int, C.c_int, C.c_void_p, C.c_double, C.c_void_p, C.c_uint64, C.c_uint64,
                                          C.c_void_p, C.c_void_p]),
+    "mcpilco_policy_backward_workspace_bytes": (C.c_size_t, [C.c_int] * 4),
+    "mcpilco_policy_backward": (C.c_int, [C.POINTER(Policy), C.c_int, C.c_int, C.c_void_p, C.c_double, C.c_void_p, C.c_uint64, C.c_uint64,
+                                          C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t,
+                                          C.c_void_p]),
     "mcpilco_init_particles": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_uint64, C.c_uint64, C.c_void_p,
                                          C.c_void_p, C.c_void_p]),
     "mcpilco_ozaki_available": (C.c_int, []),

@@ -268,9 +268,43 @@ def _workspace(dev, nbytes, tag):
     return t
 
 
-@_restores_device
 def gp_predict(gps, Xs, jac=False):
-    """Posterior mean/var [M, E] (and Jacobians [M, E, D]) of E fitted GPs at Xs.  GP_prior.py:137-155."""
+    """Posterior mean/var [M, E] (and Jacobians [M, E, D]) of E fitted GPs at Xs.  GP_prior.py:137-155.
+
+    Differentiable w.r.t. Xs (once): when grad mode is on and Xs requires grad, the forward takes the Jacobian path and the backward
+    is  dL/dXs[m] = sum_e dL/dmean[m,e] jmean[m,e] + dL/dvar[m,e] jvar[m,e].  The fitted GPs (alpha, K^-1, training inputs, kernel
+    parameters) receive no gradient.  Otherwise (and for jac=True) nothing is recorded and the outputs carry no graph."""
+    if not jac and torch.is_grad_enabled() and isinstance(Xs, torch.Tensor) and Xs.requires_grad:
+        return _GpPredict.apply(Xs, gps)
+    return _gp_predict(gps, Xs, jac)
+
+
+def gp_predict_vjp(jm, jv, g_mean, g_var):
+    """dL/dXs [M, D] from the posterior Jacobians [M, E, D] and dL/dmean, dL/dvar [M, E] (either may be None)."""
+    g = torch.zeros(jm.shape[0], jm.shape[2], dtype=F64, device=jm.device)
+    if g_mean is not None:
+        g = g + torch.einsum("me,med->md", g_mean, jm)
+    if g_var is not None:
+        g = g + torch.einsum("me,med->md", g_var, jv)
+    return g
+
+
+class _GpPredict(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, Xs, gps):
+        mean, var, jm, jv = _gp_predict(gps, Xs, jac=True)
+        ctx.save_for_backward(jm, jv)
+        return mean, var
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, g_mean, g_var):
+        jm, jv = ctx.saved_tensors
+        return gp_predict_vjp(jm, jv, g_mean, g_var), None
+
+
+@_restores_device
+def _gp_predict(gps, Xs, jac=False):
     Xs = _c(Xs, "X_test")
     L = _enter(Xs.device)
     E, M, D = len(gps), Xs.shape[0], gps[0].spec.D
@@ -414,31 +448,61 @@ def launch_count(reset=False):
     return int(N.lib().mcpilco_launch_count(1 if reset else 0))
 
 
-@_restores_device
-def policy_forward(pst, tens, x, t=0, p_dropout=0.0, masks_t=None, seed=0, particle_offset=0):
-    """u = pi(x) for a batch of states through the CUDA policy kernel.  Policy.py:242-265,323-335,389-403."""
+def _policy_call_args(pst, tens, x, t, masks_t, fn):
+    """Point the McpPolicy at the policy tensors and check the batch; returns (states, masks, tensors to keep alive)."""
     x = _c(x, "states")
-    L = _enter(x.device)
     if x.dim() != 2 or x.shape[1] != pst.Ds:
-        raise RuntimeError("policy_forward: states must be [M, %d]" % pst.Ds)
+        raise RuntimeError("%s: states must be [M, %d]" % (fn, pst.Ds))
     M = x.shape[0]
-    u = torch.empty(M, pst.Du, dtype=F64, device=x.device)
     keep = [_c(tens[k], k) for k in ("log_ls", "centers", "W")]
     pst.log_ls, pst.centers, pst.W = (k.data_ptr() for k in keep)
     b = _c(tens["bias"], "bias") if tens.get("bias") is not None else None
     tr = _c(tens["target_traj"], "target_traj") if tens.get("target_traj") is not None else None
     if tr is not None and not (0 <= int(t) < tr.shape[0]):
-        raise RuntimeError("policy_forward: time index %s outside the target trajectory" % t)
+        raise RuntimeError("%s: time index %s outside the target trajectory" % (fn, t))
     pst.bias = b.data_ptr() if b is not None else None
     pst.target_traj = tr.data_ptr() if tr is not None else None
     mk = None
     if masks_t is not None:
         mk = masks_t.detach().to(torch.uint8).contiguous()
         if not mk.is_cuda or tuple(mk.shape) != (M, pst.nb):
-            raise RuntimeError("policy_forward: masks must be a CUDA tensor [M, nb]")
+            raise RuntimeError("%s: masks must be a CUDA tensor [M, nb]" % fn)
+    return x, mk, keep + [b, tr]
+
+
+@_restores_device
+def policy_forward(pst, tens, x, t=0, p_dropout=0.0, masks_t=None, seed=0, particle_offset=0):
+    """u = pi(x) for a batch of states through the CUDA policy kernel.  Policy.py:242-265,323-335,389-403."""
+    x, mk, _keep = _policy_call_args(pst, tens, x, t, masks_t, "policy_forward")
+    L = _enter(x.device)
+    M = x.shape[0]
+    u = torch.empty(M, pst.Du, dtype=F64, device=x.device)
     N.check(L.mcpilco_policy_forward(C.byref(pst), M, int(t or 0), _ptr(x), float(p_dropout), _ptr(mk), int(seed), int(particle_offset),
                                      _ptr(u), _stream(x.device)))
     return u
+
+
+@_restores_device
+def policy_backward(pst, tens, x, g_u, t=0, p_dropout=0.0, masks_t=None, seed=0, particle_offset=0, want_gx=True):
+    """Vector-Jacobian product of policy_forward with the same arguments: {"log_ls" [1, Dp], "centers" [nb, Dp], "W" [Du, nb],
+    "bias" [Du] or None, "x" [M, Ds] or None} = g_u^T d pi(x) / d(.).  The dropout mask is the forward's (the same masks_t, or the
+    same Philox draws for the same seed and particle_offset)."""
+    x, mk, _keep = _policy_call_args(pst, tens, x, t, masks_t, "policy_backward")
+    L = _enter(x.device)
+    M, dev = x.shape[0], x.device
+    g_u = _c(g_u, "grad_u")
+    if tuple(g_u.shape) != (M, pst.Du):
+        raise RuntimeError("policy_backward: grad_u must be [%d, %d]" % (M, pst.Du))
+    out = {"log_ls": torch.empty(1, pst.Dp, dtype=F64, device=dev), "centers": torch.empty(pst.nb, pst.Dp, dtype=F64, device=dev),
+           "W": torch.empty(pst.Du, pst.nb, dtype=F64, device=dev),
+           "bias": torch.empty(pst.Du, dtype=F64, device=dev) if pst.has_bias else None,
+           "x": torch.empty(M, pst.Ds, dtype=F64, device=dev) if want_gx else None}
+    wsb = L.mcpilco_policy_backward_workspace_bytes(M, pst.nb, pst.Dp, pst.Du)
+    ws = _workspace(dev, wsb, "policy_bwd")
+    N.check(L.mcpilco_policy_backward(C.byref(pst), M, int(t or 0), _ptr(x), float(p_dropout), _ptr(mk), int(seed), int(particle_offset),
+                                      _ptr(g_u), _ptr(out["x"]), _ptr(out["log_ls"]), _ptr(out["centers"]), _ptr(out["W"]), _ptr(out["bias"]),
+                                      _ptr(ws), ws.numel(), _stream(dev)))
+    return out
 
 
 @_restores_device

@@ -153,9 +153,16 @@ class GP_prior(torch.nn.Module):
         return alpha, self.get_mean(X), K_X_inv
 
     def get_estimate_from_alpha(self, X, X_test, alpha, m_X, K_X_inv=None, Y_test=None):
-        """Posterior mean (and variance when K_X_inv is given) at X_test (reference :137-155)."""
+        """Posterior mean (and variance when K_X_inv is given) at X_test (reference :137-155).
+
+        Differentiable (once) w.r.t. X_test in both forms; the GP's parameters, X, alpha and K_X_inv receive no gradient.  With grad
+        mode on and X_test requiring grad the posterior takes the Jacobian path (the full product with K_X_inv, never the triangular
+        factor; without K_X_inv, a zero [N, N] matrix stands in for it and only the mean is returned)."""
         spec = self.gp_spec(X.shape[1])
-        if K_X_inv is None:
+        if K_X_inv is None and torch.is_grad_enabled() and X_test.requires_grad:
+            Y_hat, _ = ops.gp_predict([ops.FittedGp(spec, X, alpha, X.new_zeros(X.shape[0], X.shape[0]))], X_test)
+            var = None
+        elif K_X_inv is None:
             Y_hat = self.get_mean(X_test) + ops.gp_covariance(spec, X_test, X) @ alpha.reshape(-1, 1)
             var = None
         else:

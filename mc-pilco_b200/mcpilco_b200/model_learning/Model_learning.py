@@ -171,7 +171,8 @@ class Model_learning(torch.nn.Module):
 
     # ---- one-step prediction -----------------------------------------------------------------------------------------
     def get_exact_gp_estimate(self, gp_inputs, gp_index_list=None):
-        """Posterior mean / variance lists at gp_inputs (reference :265-289); one native call for all outputs."""
+        """Posterior mean / variance lists at gp_inputs (reference :265-289); one native call for all outputs.  Differentiable (once)
+        w.r.t. gp_inputs; the fitted GPs (alpha, K_X_inv, training inputs, hyper-parameters) receive no gradient."""
         idx = list(range(self.num_gp)) if gp_index_list is None else list(gp_index_list)
         fitted = self.fitted_gps()
         mean, var = ops.gp_predict([fitted[i] for i in idx], gp_inputs)
@@ -201,7 +202,8 @@ class Model_learning(torch.nn.Module):
         return gp_inputs, gp_outputs_list, mean_list, var_list
 
     def get_next_state(self, current_state, current_input, particle_pred=True):
-        """One model step for a batch of states (reference :210-229): variance scaled by norm**2, the mean is not."""
+        """One model step for a batch of states (reference :210-229): variance scaled by norm**2, the mean is not.  Differentiable
+        (once) w.r.t. current_state and current_input; the GPs receive no gradient."""
         _, _, mean_list, var_list = self.get_one_step_gp_out(states=current_state, inputs=current_input)
         var_list = [v * self.norm_list[i] ** 2 for i, v in enumerate(var_list)]
         return self.get_next_state_from_gp_output(current_state=current_state, current_input=current_input, gp_output_mean_list=mean_list,

@@ -6,8 +6,10 @@ Sum_of_gaussians (:153-265), Sum_of_gaussians_with_angles (:268-335), Sum_of_gau
 
 Parameter names (`log_lengthscales`, `centers`, `f_linear.weight`, `f_linear.bias`) are the reference's, so state_dicts load
 unchanged and `cost.backward()` fills the same `.grad` fields.  Inside a particle rollout the policy is evaluated by the fused
-CUDA kernels (MC_PILCO.apply_policy); calling the module on a batch of states runs the same CUDA policy kernel stand-alone
-(no autograd through a stand-alone call).  Exploration policies and PD_controller act on the real system one state at a time
+CUDA kernels (MC_PILCO.apply_policy); calling the module on a batch of states runs the same CUDA policy kernel stand-alone.
+A stand-alone call is differentiable (once) w.r.t. the parameters and the states: its backward is the CUDA vector-Jacobian product
+`torch.ops.mcpilco.policy_backward`, with the forward's dropout mask.  Under `torch.no_grad()`, or when nothing involved requires
+grad, no graph is recorded.  Exploration policies and PD_controller act on the real system one state at a time
 and are outside the hot path (SURVEY.md §2 row 7).
 """
 import numpy as np
@@ -15,6 +17,7 @@ import torch
 
 from .. import _ops as ops
 from .. import _pack as P
+from .. import torch_ops as TO
 
 
 class Policy(torch.nn.Module):
@@ -110,10 +113,18 @@ class Sum_of_gaussians(Policy):
                 "bias": self.f_linear.bias if self.flg_bias else None, "target_traj": getattr(self, "target_traj", None)}
 
     def forward(self, states, t=None, p_dropout=0.0):
-        """u = pi(states) through the CUDA policy kernel; dropout masks come from a Philox stream seeded from torch's RNG."""
+        """u = pi(states) through the CUDA policy kernel; dropout masks come from a Philox stream seeded from torch's RNG.  With grad
+        mode on and the states or a parameter requiring grad, the call is recorded for autograd (once differentiable)."""
         x = states.reshape([-1, self._raw_state_dim()])
         seed = int(torch.randint(0, 2 ** 62, (1,)).item()) if (self.flg_drop and p_dropout > 0.0) else 0
-        return ops.policy_forward(self.policy_struct(), self.policy_tensors(), x, t=0 if t is None else t, p_dropout=p_dropout, seed=seed)
+        tens = self.policy_tensors()
+        t = 0 if t is None else t
+        if torch.is_grad_enabled() and any(v is not None and v.requires_grad for v in (x, tens["log_ls"], tens["centers"], tens["W"], tens["bias"])):
+            traj = tens["target_traj"]
+            return torch.ops.mcpilco.policy_forward(TO.policy_tensor(self.policy_struct()), tens["log_ls"], tens["centers"], tens["W"],
+                                                    tens["bias"], None if traj is None else traj.detach(), x, int(t), float(p_dropout), None,
+                                                    seed, 0)
+        return ops.policy_forward(self.policy_struct(), tens, x, t=t, p_dropout=p_dropout, seed=seed)
 
 
 class Sum_of_gaussians_with_angles(Sum_of_gaussians):

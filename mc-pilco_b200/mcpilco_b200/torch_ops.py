@@ -10,6 +10,13 @@ Custom ops take tensors and scalars only, so a kernel specification travels as a
     torch.ops.mcpilco.gp_predict_jac(spec, Xtr, alpha, Kinv, Xs, var_scale) -> (mean, var, dmean/dx [M,D], dvar/dx [M,D])
     torch.ops.mcpilco.gp_nlml(spec, X, y) -> packed value + gradient (layout: include/mcpilco_b200.h)
 
+    torch.ops.mcpilco.policy_forward(pol, log_ls, centers, W, bias, target_traj, x, t, p_dropout, masks_t, seed, particle_offset) -> u
+    torch.ops.mcpilco.policy_backward(<the same arguments>, grad_u, want_gx) -> (g_log_ls, g_centers, g_W, g_bias, g_x)
+
+gp_predict and policy_forward are differentiable once (register_autograd): gp_predict w.r.t. Xs only (the fitted GP receives no
+gradient), policy_forward w.r.t. log_ls, centers, W, bias and x through policy_backward, which redraws the forward's dropout mask from
+the saved seed (or takes the same masks_t).  A policy travels as a CPU uint8 tensor with the bytes of McpPolicy (`policy_tensor`).
+
     torch.ops.mcpilco.rollout_fwd(desc, gp_specs, gp_scalars, gp_tensors, log_ls, centers, W, bias, policy_traj, cost_traj, x0,
                                   eps, masks, meas_eps, seed_dev, need_grad) -> (states, inputs, cost[2], cost_stats[H,2], jac, pol_in)
     torch.ops.mcpilco.rollout_bwd(<the same leading arguments>, states, inputs, jac, pol_in, grad_cost, grad_states, grad_inputs,
@@ -60,14 +67,14 @@ def gp_precompute(spec: torch.Tensor, X: torch.Tensor, y: torch.Tensor) -> Tuple
 @torch.library.custom_op("mcpilco::gp_predict", mutates_args=(), device_types="cuda")
 def gp_predict(spec: torch.Tensor, Xtr: torch.Tensor, alpha: torch.Tensor, Kinv: torch.Tensor, Xs: torch.Tensor,
                var_scale: float) -> Tuple[torch.Tensor, torch.Tensor]:
-    mean, var = ops.gp_predict([ops.FittedGp(_spec(spec), Xtr, alpha, Kinv, var_scale=var_scale)], Xs)
+    mean, var = ops._gp_predict([ops.FittedGp(_spec(spec), Xtr, alpha, Kinv, var_scale=var_scale)], Xs)
     return mean, var
 
 
 @torch.library.custom_op("mcpilco::gp_predict_jac", mutates_args=(), device_types="cuda")
 def gp_predict_jac(spec: torch.Tensor, Xtr: torch.Tensor, alpha: torch.Tensor, Kinv: torch.Tensor, Xs: torch.Tensor,
                    var_scale: float) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
-    mean, var, jm, jv = ops.gp_predict([ops.FittedGp(_spec(spec), Xtr, alpha, Kinv, var_scale=var_scale)], Xs, jac=True)
+    mean, var, jm, jv = ops._gp_predict([ops.FittedGp(_spec(spec), Xtr, alpha, Kinv, var_scale=var_scale)], Xs, jac=True)
     return mean, var, jm[:, 0, :].contiguous(), jv[:, 0, :].contiguous()
 
 
@@ -105,6 +112,94 @@ def _(spec, Xtr, alpha, Kinv, Xs, var_scale):
 @gp_nlml.register_fake
 def _(spec, X, y):
     return X.new_empty(4 + N.MAX_D + N.MAX_POLY * N.MAX_DEG * (N.MAX_D + 1))
+
+
+def _no_double_backward(name):
+    if torch.is_grad_enabled():
+        raise RuntimeError("mcpilco: %s is differentiable once; double backward (create_graph=True) is not supported" % name)
+
+
+# d/dXs of the posterior (the fitted GP itself receives no gradient): the backward recomputes the Jacobians through gp_predict_jac
+def _gp_predict_setup(ctx, inputs, output):
+    ctx.args = inputs
+
+
+def _gp_predict_backward(ctx, g_mean, g_var):
+    _no_double_backward("mcpilco::gp_predict")
+    spec, Xtr, alpha, Kinv, Xs, var_scale = ctx.args
+    if not ctx.needs_input_grad[4]:
+        return None, None, None, None, None, None
+    _, _, jm, jv = gp_predict_jac(spec, Xtr, alpha, Kinv, Xs, var_scale)
+    return None, None, None, None, ops.gp_predict_vjp(jm.unsqueeze(1), jv.unsqueeze(1), g_mean, g_var), None
+
+
+gp_predict.register_autograd(_gp_predict_backward, setup_context=_gp_predict_setup)
+
+
+# ---------------------------------------------------------------------------------------------------------------------
+# the stand-alone policy (Sum_of_gaussians.forward, Policy.py:242-265,323-335,389-403) and its vector-Jacobian product
+# ---------------------------------------------------------------------------------------------------------------------
+def policy_tensor(pst):
+    """CPU uint8 tensor with the bytes of a McpPolicy (its pointer fields are re-pointed at the tensor arguments on every call)."""
+    return torch.frombuffer(bytearray(_bytes_of(pst)), dtype=torch.uint8).clone()
+
+
+def _policy(t):
+    if t.device.type != "cpu" or t.dtype != torch.uint8 or t.numel() != C.sizeof(N.Policy):
+        raise RuntimeError("mcpilco: policy must be a CPU uint8 tensor of %d bytes (torch_ops.policy_tensor)" % C.sizeof(N.Policy))
+    return N.Policy.from_buffer_copy(bytes(t.contiguous().numpy().tobytes()))
+
+
+def _ptens(log_ls, centers, W, bias, target_traj):
+    return {"log_ls": log_ls, "centers": centers, "W": W, "bias": bias, "target_traj": target_traj}
+
+
+@torch.library.custom_op("mcpilco::policy_forward", mutates_args=(), device_types="cuda")
+def policy_forward(pol: torch.Tensor, log_ls: torch.Tensor, centers: torch.Tensor, W: torch.Tensor, bias: Optional[torch.Tensor],
+                   target_traj: Optional[torch.Tensor], x: torch.Tensor, t: int, p_dropout: float, masks_t: Optional[torch.Tensor],
+                   seed: int, particle_offset: int) -> torch.Tensor:
+    return ops.policy_forward(_policy(pol), _ptens(log_ls, centers, W, bias, target_traj), x, t=t, p_dropout=p_dropout, masks_t=masks_t,
+                              seed=seed, particle_offset=particle_offset)
+
+
+@torch.library.custom_op("mcpilco::policy_backward", mutates_args=(), device_types="cuda")
+def policy_backward(pol: torch.Tensor, log_ls: torch.Tensor, centers: torch.Tensor, W: torch.Tensor, bias: Optional[torch.Tensor],
+                    target_traj: Optional[torch.Tensor], x: torch.Tensor, t: int, p_dropout: float, masks_t: Optional[torch.Tensor],
+                    seed: int, particle_offset: int, grad_u: torch.Tensor,
+                    want_gx: bool) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
+    g = ops.policy_backward(_policy(pol), _ptens(log_ls, centers, W, bias, target_traj), x, grad_u, t=t, p_dropout=p_dropout, masks_t=masks_t,
+                            seed=seed, particle_offset=particle_offset, want_gx=want_gx)
+    none = lambda: x.new_empty(0)  # noqa: E731
+    return g["log_ls"], g["centers"], g["W"], g["bias"] if g["bias"] is not None else none(), g["x"] if g["x"] is not None else none()
+
+
+@policy_forward.register_fake
+def _(pol, log_ls, centers, W, bias, target_traj, x, t, p_dropout, masks_t, seed, particle_offset):
+    return x.new_empty(x.shape[0], W.shape[0])
+
+
+@policy_backward.register_fake
+def _(pol, log_ls, centers, W, bias, target_traj, x, t, p_dropout, masks_t, seed, particle_offset, grad_u, want_gx):
+    e = x.new_empty
+    return e(log_ls.shape), e(centers.shape), e(W.shape), e(W.shape[0] if bias is not None else 0), e(x.shape if want_gx else 0)
+
+
+def _policy_setup(ctx, inputs, output):
+    ctx.args = inputs  # the seed among them: the backward redraws the forward's Philox dropout mask
+
+
+def _policy_backward(ctx, grad_u):
+    _no_double_backward("mcpilco::policy_forward")
+    pol, log_ls, centers, W, bias, target_traj, x, t, p_dropout, masks_t, seed, particle_offset = ctx.args
+    need = ctx.needs_input_grad
+    gl, gc, gw, gb, gx = policy_backward(pol, log_ls.detach(), centers.detach(), W.detach(), None if bias is None else bias.detach(),
+                                         target_traj, x.detach(), t, p_dropout, masks_t, seed, particle_offset, grad_u.contiguous(),
+                                         bool(need[6]))
+    return (None, gl.reshape(log_ls.shape) if need[1] else None, gc if need[2] else None, gw if need[3] else None,
+            gb if (bias is not None and need[4]) else None, None, gx.reshape(x.shape) if need[6] else None, None, None, None, None, None)
+
+
+policy_forward.register_autograd(_policy_backward, setup_context=_policy_setup)
 
 
 # ---------------------------------------------------------------------------------------------------------------------
