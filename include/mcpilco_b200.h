@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define MCP_ABI_VERSION 7
+#define MCP_ABI_VERSION 8
 
 #define MCP_MAX_D 32    /* gp-input dimension            */
 #define MCP_MAX_DS 16   /* state dimension               */
@@ -289,9 +289,14 @@ int mcpilco_prof_read(double* total_ms, uint64_t* launches, double* flops);
  * segments of at most 65536 / slices columns (exact int32 accumulation), recombined in fp64. */
 int mcpilco_ozaki_available(void);
 size_t mcpilco_ozaki_plane_bytes(int N, int slices);
+/* prepare(): exponents[n] is the power of two of row n's scale, ilogb(max_k |Kinv[n][k]|) + 3 (0 for a zero row), or
+ * MCP_OZAKI_EXP_NONFINITE when the row holds a NaN or an infinity; such a row gets zero digits. */
+#define MCP_OZAKI_EXP_NONFINITE 1048576
 int mcpilco_ozaki_prepare(const double* Kinv, int N, int ld, int slices, int8_t* planes, int32_t* exponents, void* stream);
 /* the contraction on its own: V[M, N] (ldv) = A[M, N] (lda) * Kinv^T from Kinv's prepared planes (used by mcpilco_gp_predict /
- * mcpilco_rollout_fwd when McpGp.ozaki_slices != 0; exported for tests and benchmarks) */
+ * mcpilco_rollout_fwd when McpGp.ozaki_slices != 0; exported for tests and benchmarks).  A NaN or an infinity in row m of A makes row
+ * m of V NaN, one in row n of Kinv (exponent MCP_OZAKI_EXP_NONFINITE) makes column n of V NaN; every other element is unaffected.
+ * Only columns [0, N) of the rows of A and V are read or written. */
 size_t mcpilco_ozaki_scratch_bytes(int M, int N, int slices);
 int mcpilco_ozaki_contract(const double* A, int lda, int M, int N, int slices, const int8_t* planes, const int32_t* exponents, double* V,
                            int ldv, void* scratch, size_t scratch_bytes, void* stream);

@@ -24,18 +24,25 @@ namespace mcp {
 // ---- slicing: one warp per row -----------------------------------------------------------------------------------
 // The contraction index is cut into `nseg` segments of Ks columns (S * Ks <= 65536 keeps every int32 plane product exact); a segment's
 // planes are contiguous:  planes[row][seg][p][k],  p = t (reverse == 0) or S-1-t (reverse == 1), k < Ksp (Ks rounded up to 128, zero
-// padded).  Row stride nseg * S * Ksp bytes.  One exponent per row, common to all segments.
+// padded).  Row stride nseg * S * Ksp bytes.  One exponent per row, common to all segments; a row with a NaN or an infinity gets the
+// exponent MCP_OZAKI_EXP_NONFINITE and zero digits, and the contraction's epilogue writes NaN wherever that row meets the product.
 __global__ void __launch_bounds__(256) ozaki_slice_kernel(const double* __restrict__ A, int rows, int K, int ld, int S, int Ks, int Ksp, int nseg,
                                                           int reverse, int8_t* __restrict__ planes, int32_t* __restrict__ expo) {
   const int row = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
   if (row >= rows) return;
   const double* a = A + (size_t)row * ld;
   double mx = 0.0;
-  for (int k = lane; k < K; k += 32) mx = fmax(mx, fabs(a[k]));
+  bool finite = true;
+  for (int k = lane; k < K; k += 32) {
+    const double v = a[k];
+    finite = finite && isfinite(v);
+    mx = fmax(mx, fabs(v));
+  }
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, o));
-  const int e = (mx > 0.0 && isfinite(mx)) ? ilogb(mx) + 3 : 0;  // |a| 2^-e < 1/4: the most significant balanced digit stays within
-                                                                   // [-65, 65] after the carries from below (no wrap at +128)
+  finite = __all_sync(0xffffffffu, finite);
+  // |a| 2^-e < 1/4: the most significant balanced digit stays within [-65, 65] after the carries from below (no wrap at +128)
+  const int e = !finite ? MCP_OZAKI_EXP_NONFINITE : mx > 0.0 ? ilogb(mx) + 3 : 0;
   if (lane == 0) expo[row] = e;
   int8_t* out = planes + (size_t)row * nseg * S * Ksp;
   const int sh = 8 * S - e;
@@ -46,10 +53,7 @@ __global__ void __launch_bounds__(256) ozaki_slice_kernel(const double* __restri
 #pragma unroll
     for (int i = 0; i < 4; i++) {
       F[i] = 0;
-      if (k + i < Ks && col + i < K) {
-        const double v = a[col + i];
-        F[i] = isfinite(v) ? __double2ll_rn(scalbn(v, sh)) : 0;  // |F| < 2^(8S-2) <= 2^62
-      }
+      if (finite && k + i < Ks && col + i < K) F[i] = __double2ll_rn(scalbn(a[col + i], sh));  // |F| < 2^(8S-2) <= 2^62
     }
     // balanced base-256 digits without a carry chain: F = sum_t d_t 256^t with d_t in [-128, 127]  <=>  F + sum_t 128 256^t has the
     // plain bytes d_t + 128, and (byte ^ 0x80) is d_t as int8.  Plane p holds digit t = S-1-p (most significant digit in plane 0).

@@ -410,9 +410,13 @@ ozaki_mma_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
                   for (int j = 0; j < 16; j++) v[j] = fma((double)r[a][j], sc, v[j]);
                 }
               }
-              if (last) {
+              if (last) {  // row / column scales; a row of A or of B marked non-finite by the slicer makes the element NaN (finite
+                           // rows have exponents within +-1100, so a sum above half the marker holds one)
 #pragma unroll
-                for (int j = 0; j < 16; j++) v[j] = scalbn(v[j], ea + (col0 + j < N ? eB[col0 + j] : 0));
+                for (int j = 0; j < 16; j++) {
+                  const int ex = ea + (col0 + j < N ? eB[col0 + j] : 0);
+                  v[j] = ex > MCP_OZAKI_EXP_NONFINITE / 2 ? __longlong_as_double(0x7FF8000000000000ll) : scalbn(v[j], ex);
+                }
               }
               if (vec) {
 #pragma unroll

@@ -6,7 +6,8 @@ import ctypes as C
 import os
 
 MAX_D, MAX_DS, MAX_DU, MAX_E, MAX_DP, MAX_POLY, MAX_DEG = 32, 16, 8, 16, 32, 3, 3
-ABI_VERSION = 7
+ABI_VERSION = 8
+OZAKI_EXP_NONFINITE = 1 << 20  # row exponent of the INT8 contraction's digit planes for a row with a NaN / inf
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libmcpilco_b200.so")
 

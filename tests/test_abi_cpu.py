@@ -37,7 +37,8 @@ def test_header_limits_match_binding(native):
     hdr = open(os.path.join(ROOT, "include", "mcpilco_b200.h")).read()
     for name, val in (("MCP_MAX_D", native.MAX_D), ("MCP_MAX_DS", native.MAX_DS), ("MCP_MAX_DU", native.MAX_DU),
                       ("MCP_MAX_E", native.MAX_E), ("MCP_MAX_DP", native.MAX_DP), ("MCP_MAX_POLY", native.MAX_POLY),
-                      ("MCP_MAX_DEG", native.MAX_DEG), ("MCP_ABI_VERSION", native.ABI_VERSION)):
+                      ("MCP_MAX_DEG", native.MAX_DEG), ("MCP_ABI_VERSION", native.ABI_VERSION),
+                      ("MCP_OZAKI_EXP_NONFINITE", native.OZAKI_EXP_NONFINITE)):
         assert int(re.search(r"#define\s+%s\s+(\d+)" % name, hdr).group(1)) == val
 
 
